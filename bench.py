@@ -246,6 +246,31 @@ def workload_config(n_gpus):
             "l2": "inputs (128 MiB of tuples per GPU) exceed the 126 MB L2; no flush needed"}
 
 
+DUMP_BYTES_MAX = 64 * 10**6
+
+
+def dump_outputs(out_dir, bitmap_words, results, n_items, result_dtype):
+    """Writes what a caller of the timed path receives from its last step, so that two builds can be compared output for
+    output on identical inputs (the tiled config-3 fixture: nothing in the timed path's inputs is random):
+      verdicts.npy       float32, the 0/1 verdict of every tuple; when that would exceed the 64 MB budget, a fixed seeded sample
+                         of the tuples, whose indices are in verdicts_index.npy (float64)
+      quorum_counts.npy  float64 (groups, 3): n_valid, n_distinct, has_quorum of every group
+      quorum_power.npy   float64 (groups, 10): the 320-bit voted power of every group as little-endian 32-bit limbs (exact)"""
+    os.makedirs(out_dir, exist_ok=True)
+    bits = np.unpackbits(bitmap_words.cpu().numpy().view(np.uint8), bitorder="little")[:n_items]
+    res = results.cpu().numpy().view(result_dtype)
+    counts = np.stack([res["n_valid"], res["n_distinct"], res["has_quorum"]], axis=1).astype(np.float64)
+    power = np.ascontiguousarray(res["power"]).view(np.uint32).astype(np.float64)
+    budget = DUMP_BYTES_MAX - counts.nbytes - power.nbytes - 4 * 4096   # room for the .npy headers
+    if 4 * n_items > budget:
+        idx = np.sort(np.random.default_rng(0).choice(n_items, budget // 12, replace=False))  # 4 B verdict + 8 B index each
+        bits = bits[idx]
+        np.save(os.path.join(out_dir, "verdicts_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(out_dir, "verdicts.npy"), bits.astype(np.float32))
+    np.save(os.path.join(out_dir, "quorum_counts.npy"), counts)
+    np.save(os.path.join(out_dir, "quorum_power.npy"), power)
+
+
 def _pct(xs, q):
     xs = sorted(xs)
     return xs[min(len(xs) - 1, int(len(xs) * q))] if xs else None
@@ -595,7 +620,12 @@ def main():
     ap.add_argument("--no-key-cache-leg", action="store_true", help="skip the extra leg that times the key-registry path")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--skip-extras", action="store_true", help="headline + e2e + strong-scaling legs only (development: short multi-GPU runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the verdicts and quorum results of the last timed step to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)
@@ -717,6 +747,8 @@ def main():
         sampler.stop()
     ms_per_step = ms_total / args.steps
     value = n_global / (ms_per_step * 1e-3)
+    if args.dump_outputs and rank == 0:   # before any later leg writes t_results again
+        dump_outputs(args.dump_outputs, full_bitmap(), t_results, n_global, ib.RESULT_DTYPE)
 
     # ---- e2e: host buffers through ibft_verify_batch (H2D + kernels + D2H inside the timed region)
     # the step's inputs live in PINNED host memory (torch pin_memory); the C ABI detects that and DMA-copies straight from it
