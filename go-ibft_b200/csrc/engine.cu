@@ -1646,6 +1646,7 @@ struct lane {
   pending_call pending;
   uint32_t* d_worklist = nullptr;  // key-registry path: [0] = count, [1..] = indices left to the recover pass
   cudaEvent_t wl_ev[4] = {nullptr, nullptr, nullptr, nullptr};  // last use of each worklist (orders launches that arrive on different streams)
+  uint32_t wl_used = 0;  // bit k: worklist k was filled by the current / last host-buffer call (ibft_debug_last_deferred)
   const uint8_t* dev_arena = nullptr;
   size_t dev_arena_len = 0;
 };
@@ -1800,15 +1801,17 @@ static int engine_alloc(ibft_engine* e) {
   return IBFT_OK;
 }
 
-// test hook: copy `count` entries of the combined generator table starting at entry `first` (64 bytes each, x then y as 8
-// little-endian words); returns IBFT_ERR_INVALID_ARG when the library was built without a combined table
+// test hook: copy `count` entries of the generator comb starting at entry `first` (64 bytes each, x then y as 8 little-endian
+// words).  The positions lie back to back on the device (load_comb_pos): entry index = position * IBFT_CTAB_ENTRIES + in-position
+// index, for every one of the IBFT_CTAB_POSITIONS positions.  Returns IBFT_ERR_INVALID_ARG when the library was built without a
+// combined table
 extern "C" int ibft_debug_ctable(ibft_engine* e, uint32_t first, uint32_t count, uint8_t* out, int* wc, uint32_t* entries) {
   if (!e) { set_err("null engine"); return IBFT_ERR_INVALID_ARG; }
   if (wc) *wc = IBFT_WC;
 #if IBFT_WC > 0
   if (entries) *entries = (uint32_t)IBFT_CTAB_ENTRIES;
   if (count == 0) return IBFT_OK;
-  if (!out || (size_t)first + count > (size_t)IBFT_CTAB_ENTRIES) { set_err("range"); return IBFT_ERR_INVALID_ARG; }
+  if (!out || (size_t)first + count > (size_t)IBFT_CTAB_POSITIONS * IBFT_CTAB_ENTRIES) { set_err("range"); return IBFT_ERR_INVALID_ARG; }
   CU(cudaSetDevice(e->p.device));
   CU(cudaMemcpy(out, e->d_ctable + (size_t)first * IBFT_GTAB_ENTRY_WORDS, (size_t)count * 64, cudaMemcpyDeviceToHost));
   return IBFT_OK;
@@ -1817,6 +1820,29 @@ extern "C" int ibft_debug_ctable(ibft_engine* e, uint32_t first, uint32_t count,
   (void)first; (void)out;
   return count == 0 ? IBFT_OK : IBFT_ERR_INVALID_ARG;
 #endif
+}
+
+// test hook: copy `count` entries of validator `validator`'s key table in `slot` (entry index = position * IBFT_KEYTAB_ENTRIES +
+// m - 1 holds m * 2^(8 position) * Q; same 64-byte format as ibft_debug_ctable) and its registry state
+extern "C" int ibft_debug_keytab(ibft_engine* e, uint32_t slot, uint32_t validator, uint32_t first, uint32_t count, uint8_t* out,
+                                 uint32_t* state_out) {
+  if (!e) { set_err("null engine"); return IBFT_ERR_INVALID_ARG; }
+  all_lanes_lock lk(e);
+  if (slot >= e->p.max_table_slots || !e->slots[slot].valid) { set_err("slot %u not set", slot); return IBFT_ERR_NO_TABLE; }
+  const slot_host& s = e->slots[slot];
+  if (!s.d_key_state || validator >= s.n) { set_err("no key registry entry %u in slot %u", validator, slot); return IBFT_ERR_INVALID_ARG; }
+#if IBFT_WC > 0
+  if (count && (!out || (size_t)first + count > (size_t)IBFT_KEYTAB_WORDS / IBFT_GTAB_ENTRY_WORDS)) { set_err("range"); return IBFT_ERR_INVALID_ARG; }
+  CU(cudaSetDevice(e->p.device));
+  CU(cudaDeviceSynchronize());
+  if (state_out) CU(cudaMemcpy(state_out, s.d_key_state + validator, 4, cudaMemcpyDeviceToHost));
+  if (count)
+    CU(cudaMemcpy(out, s.d_key_tab + (size_t)validator * IBFT_KEYTAB_WORDS + (size_t)first * IBFT_GTAB_ENTRY_WORDS, (size_t)count * 64,
+                  cudaMemcpyDeviceToHost));
+#else
+  (void)first; (void)count; (void)out; (void)state_out;
+#endif
+  return IBFT_OK;
 }
 
 extern "C" int ibft_engine_create(const ibft_engine_params* params, ibft_engine** out) {
@@ -2144,6 +2170,7 @@ static int launch_recover(ibft_engine* e, lane* L, const ibft_sig_item* d_items,
     uint32_t blocks = (cnt + IBFT_SPLIT_SIGS - 1) / IBFT_SPLIT_SIGS;
     CU(cudaStreamWaitEvent(st, L->wl_ev[worklist_index & 3u], 0));
     CU(cudaMemsetAsync(worklist, 0, 4, st));
+    L->wl_used |= 1u << (worklist_index & 3u);
     k_verify_split<<<blocks, 32 * (IBFT_SPLIT_CHAINS + 1), IBFT_VSPLIT_SMEM, st>>>(d_items, n, d_arena, arena_len, lo, hi, d_groups, n_groups,
                                                                               e->d_slots, e->p.max_table_slots, d_bitmap, d_status, e->d_ctable,
                                                                               sink, worklist);
@@ -2172,6 +2199,7 @@ static int launch_recover(ibft_engine* e, lane* L, const ibft_sig_item* d_items,
     // device-resident callers may use different streams: launches sharing a worklist are ordered on the device
     CU(cudaStreamWaitEvent(st, L->wl_ev[worklist_index & 3u], 0));
     CU(cudaMemsetAsync(worklist, 0, 4, st));
+    L->wl_used |= 1u << (worklist_index & 3u);
     if (small_batch) {
       k_verify_known<32><<<(cnt + 31) / 32, 32, 0, st>>>(d_items, n, d_arena, arena_len, lo, hi, d_groups, n_groups, e->d_slots,
                                                         e->p.max_table_slots, d_bitmap, d_status, e->d_ctable, sink, worklist);
@@ -2270,6 +2298,7 @@ static int submit_locked(ibft_engine* e, lane* L, const ibft_sig_item* items, ui
     L->last_groups.clear();
   }
   cudaStream_t st = L->stream;
+  L->wl_used = 0;
   if (arena_len) {
     memcpy(L->h_arena, arena, arena_len);
     CU(cudaMemcpyAsync(L->d_arena, L->h_arena, arena_len, cudaMemcpyHostToDevice, st));
@@ -2490,6 +2519,25 @@ extern "C" int ibft_last_item_status(ibft_engine* e, uint8_t* status_out, uint32
   if (L->pending.active) { set_err("a submitted call is still pending"); return IBFT_ERR_INVALID_ARG; }
   if (n > L->last_status_n) { set_err("last call had %u items", L->last_status_n); return IBFT_ERR_INVALID_ARG; }
   memcpy(status_out, L->h_status, n);
+  return IBFT_OK;
+}
+
+// test hook: items the known-key pass of the most recent completed host-buffer call left to the recover pass -- the sum of the
+// counts of the worklists that call filled.  Exact for calls of at most two chunks (2^18 items): a third chunk re-uses a list.
+extern "C" int ibft_debug_last_deferred(ibft_engine* e, uint32_t* count) {
+  if (!e || !count) { set_err("null argument"); return IBFT_ERR_INVALID_ARG; }
+  lane* L = &e->lanes[e->last_lane.load()];
+  std::lock_guard<std::mutex> lk(L->mu);
+  if (L->pending.active) { set_err("a submitted call is still pending"); return IBFT_ERR_INVALID_ARG; }
+  *count = 0;
+  if (!L->d_worklist) return IBFT_OK;
+  CU(cudaSetDevice(e->p.device));
+  for (uint32_t k = 0; k < 4; k++) {
+    if (!((L->wl_used >> k) & 1u)) continue;
+    uint32_t c = 0;
+    CU(cudaMemcpy(&c, L->d_worklist + (size_t)k * ((size_t)L->cap_items + 1), 4, cudaMemcpyDeviceToHost));
+    *count += c;
+  }
   return IBFT_OK;
 }
 

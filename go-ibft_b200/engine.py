@@ -34,6 +34,7 @@ EXPORTS = [
     "ibft_verify_wait", "ibft_bind_groups", "ibft_verify_batch_device", "ibft_quorum_reduce_device", "ibft_quorum_partial_words", "ibft_quorum_mark_device", "ibft_quorum_merge_device", "ibft_quorum_exchange_device",
     "ibft_exchange_alloc", "ibft_exchange_open", "ibft_exchange_close", "ibft_exchange_free", "ibft_exchange_clear",
     "ibft_get_voted_bitmap", "ibft_keccak256_batch", "ibft_proposal_hash_batch", "ibft_sign_batch", "ibft_engine_launch_count", "ibft_set_recover_path", "ibft_refresh_key_tables", "ibft_probe_int_peak", "ibft_debug_op", "ibft_debug_ctable",
+    "ibft_debug_keytab", "ibft_debug_last_deferred",
 ]
 
 
@@ -103,6 +104,8 @@ def load_library(path: str | None = None) -> ctypes.CDLL:
     lib.ibft_probe_int_peak.argtypes = [c_void_p, POINTER(c_double), POINTER(c_double)]
     lib.ibft_debug_ctable.argtypes = [c_void_p, c_uint32, c_uint32, c_void_p, POINTER(c_int), POINTER(c_uint32)]
     lib.ibft_debug_op.argtypes = [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_uint32, c_void_p, c_uint32]
+    lib.ibft_debug_keytab.argtypes = [c_void_p, c_uint32, c_uint32, c_uint32, c_uint32, c_void_p, POINTER(c_uint32)]
+    lib.ibft_debug_last_deferred.argtypes = [c_void_p, POINTER(c_uint32)]
     if path is None:
         _LIB = lib
     return lib
@@ -359,9 +362,23 @@ class Engine:
         return int(wc.value), int(n.value)
 
     def combined_table_entries(self, first: int, count: int) -> np.ndarray:
+        """entries [first, first + count) of the generator comb, all positions back to back (x, y as 8 little-endian words)"""
         out = np.zeros((count, 16), dtype=np.uint32)
         self._check(self.lib.ibft_debug_ctable(self.handle, first, count, _ptr(out), None, None))
         return out
+
+    def key_table_entries(self, slot: int, validator: int, first: int = 0, count: int = 0):
+        """(registry state, entries [first, first + count) of a validator's key comb): entry j * 128 + m - 1 = m * 2^(8j) * Q"""
+        out = np.zeros((count, 16), dtype=np.uint32)
+        st = c_uint32()
+        self._check(self.lib.ibft_debug_keytab(self.handle, slot, validator, first, count, _ptr(out) if count else None, ctypes.byref(st)))
+        return int(st.value), out
+
+    def last_deferred(self) -> int:
+        """items the known-key pass of the last completed host-buffer call left to the recover pass"""
+        c = c_uint32()
+        self._check(self.lib.ibft_debug_last_deferred(self.handle, ctypes.byref(c)))
+        return int(c.value)
 
     # ---- primitive parity hooks (tests)
     def debug_op(self, op: str, a: list[int], b: list[int] | None = None, c: list[bytes] | None = None, out_stride: int = 32):

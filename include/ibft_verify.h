@@ -314,10 +314,21 @@ int ibft_probe_int_peak(ibft_engine* e, double* imad_per_s, double* wide_mac_per
 #define IBFT_DBG_FE_ADD 8   /* out = a+b mod p */
 #define IBFT_DBG_FE_SUB 9   /* out = a-b mod p */
 #define IBFT_DBG_GLV 10     /* out(64) = |k1| (16B BE) || |k2| (16B BE) || sign1 || sign2 padded -- see tests */
-/* Combined generator table (builds with IBFT_WC > 0): *wc = window (0 when absent), *entries = table size; copies `count`
- * 64-byte entries (x, y as 8 little-endian words each) starting at `first`.  Entry index = d1 * (2^wc + 1) + d2 + 2^(wc-1)
- * holds d1*G + d2*lambda*G. */
+/* Combined generator table (builds with IBFT_WC > 0): *wc = window (0 when absent), *entries = entries of ONE comb position;
+ * copies `count` 64-byte entries (x, y as 8 little-endian words each) starting at `first`.  The comb positions j = 0, 1, ...
+ * (17 for wc = 8) follow one another: entry index = j * entries + d1 * (2^wc + 1) + d2 + 2^(wc-1) holds
+ * 2^(wc j) * (d1*G + d2*lambda*G); first + count may run up to the end of the last position. */
 int ibft_debug_ctable(ibft_engine* e, uint32_t first, uint32_t count, uint8_t* out, int* wc, uint32_t* entries);
+/* Key registry (IBFT_FLAG_KEY_CACHE, tests only): copies `count` 64-byte entries (same format) of the comb table of validator
+ * `validator` (validator-index order) of table slot `slot`, starting at `first`: entry index = j * 128 + m - 1 holds
+ * m * 2^(8 j) * Q for comb position j and m = 1..128.  *state_out (may be NULL): 0 key unknown, 1 learned, 3 table being
+ * built, 2 table READY (only a READY table is ever read by the verification). */
+int ibft_debug_keytab(ibft_engine* e, uint32_t slot, uint32_t validator, uint32_t first, uint32_t count, uint8_t* out,
+                      uint32_t* state_out);
+/* Key registry (tests only): *count = number of items that the known-key pass of the most recent completed host-buffer call
+ * left to the recover pass (key not ready, or the verification against the key rejected).  0 when that call took no
+ * known-key pass.  Exact for calls of at most 2^18 items (two upload chunks; a third chunk re-uses a worklist). */
+int ibft_debug_last_deferred(ibft_engine* e, uint32_t* count);
 int ibft_debug_op(ibft_engine* e, int op, const uint8_t* a, const uint8_t* b, const uint8_t* c, uint32_t n,
                   uint8_t* out, uint32_t out_stride);
 
